@@ -16,17 +16,21 @@ compaction, stats (config 2: followed by ground_water_augmentation(water_height 
 device).  With N > 1 every rank augments its own 32 clouds (clouds are independent, no data-path collective) and one
 all-gather reassembles the augmented batch on every rank (configs[3]).
 
-`value`     device-resident inputs.  A bracket = EXACTLY K steps between one CUDA-event pair on the launching stream
-            (barrier + synchronize on both sides, max over ranks); the bracket is repeated until >= 1 s of device time has
-            been measured and the MEDIAN bracket is reported (`repeats`, `ms_per_step_min/max` beside it).  Two input
-            batches alternate so that no step finds its rows in L2.
+`value`     device-resident inputs.  The K timed steps run as one bracket between one CUDA-event pair on the launching
+            stream (barrier + synchronize on both sides, max over ranks).  Two input batches alternate so that no step
+            finds its rows in L2.
 `e2e`       the public API with pinned HOST buffers: H2D of the batch + augment + D2H of the augmented batch, per step
+            (K pipelined steps, then K synchronous calls)
 `roofline`  the beam stage (scan + solve kernels) against the measured HBM copy peak; algorithmic bytes per launch =
             40 B x points + 12 B x table particles (SURVEY.md 8d), durations from CUDA events on the launching stream
 `cpu_baseline` / --impl reference
             the CPU oracle port (oracle/) on all host cores: one worker process per cloud (4 threads each for its 64
             channel tasks), 32 clouds per step, median step; tables from the oracle's own dart throwing -- this arm never
             loads the product library
+
+--dump-outputs DIR writes what the last timed step returned as DIR/<name>.npy (float32 / float64): every per-cloud
+array in full and, of the augmented rows, the kept rows of a fixed seeded sample of clouds (`points_clouds`), < 64 MB in
+all.  The inputs depend only on the arguments, so two builds can be compared output for output.
 """
 import argparse
 import json
@@ -43,6 +47,7 @@ import numpy as np
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark writes nothing into the tree it runs from (it may be read-only)
 
 SNOWFALL_RATE = 2.5
 TERMINAL_VELOCITY = 1.6
@@ -57,7 +62,7 @@ ALGO_BYTES_PER_PARTICLE = 12        # f32 x, y, r once per launch (SURVEY.md 8d)
 FIXED_POLY = (2e-3, -0.3, 12.0)     # only used with --host-threshold
 CPU_CLOUDS_PER_STEP = 32
 CPU_THREADS_PER_CLOUD = 4
-MIN_TIMED_MS = 1000.0
+DUMP_POINTS_BYTES = 48 << 20        # --dump-outputs: budget of the sampled kept rows (the per-cloud arrays are small)
 STEPS_IN_FLIGHT = 1                 # device-resident leg: consecutive steps on alternating streams (1 = strictly serial)
 
 
@@ -283,6 +288,23 @@ def run_reference(args):
 # ----------------------------------------------------------------------------------------------------------------------
 # our arm
 # ----------------------------------------------------------------------------------------------------------------------
+def dump_outputs(out_dir, res, off, seed=0):
+    """Write one step's result dict as <out_dir>/<name>.npy: the per-cloud arrays in full (float64), and of the
+    slot-compacted rows `points` only the kept rows of a fixed seeded sample of clouds that fits DUMP_POINTS_BYTES
+    (float32, concatenated in cloud order; the clouds in `points_clouds`)."""
+    os.makedirs(out_dir, exist_ok=True)
+    counts = res['counts'].cpu().numpy().astype(np.int64)
+    n_per = np.diff(off)
+    n_clouds = min(len(n_per), DUMP_POINTS_BYTES // (20 * int(n_per.max())))
+    clouds = np.sort(np.random.default_rng(seed).choice(len(n_per), n_clouds, replace=False))
+    pts = res['points']
+    arrays = {'points': np.concatenate([pts[off[b]:off[b] + counts[b]].cpu().numpy() for b in clouds]),
+              'points_clouds': clouds.astype(np.float64)}
+    arrays.update({name: t.cpu().numpy().astype(np.float64) for name, t in res.items() if name != 'points'})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, f'{name}.npy'), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
@@ -298,7 +320,8 @@ def main():
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
     ap.add_argument('--no-gather', action='store_true', help='N > 1: replicas only, skip the all-gather (debug)')
-    ap.add_argument('--min-timed-ms', type=float, default=MIN_TIMED_MS)
+    ap.add_argument('--dump-outputs', metavar='DIR', default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (rank 0's batch)")
     ap.add_argument('--streams', type=int, default=STEPS_IN_FLIGHT, choices=[1, 2],
                     help='steps in flight in the device-resident leg: consecutive steps alternate between this many streams')
     ap.add_argument('--e2e-inflight', type=int, default=3, help='batches in flight in the e2e leg (1..3)')
@@ -454,24 +477,20 @@ def main():
         step(k)
     drain()
     eng.check()
-    est = bracket(args.steps)                               # untimed estimate: how many brackets make >= 1 s
-    repeats = int(min(400, max(3, np.ceil(args.min_timed_ms / max(est, 1e-3)))))
-    if world > 1:
-        t = torch.tensor([repeats], dtype=torch.int64, device=dev)
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)
-        repeats = int(t.item())
     launches0 = eng.launch_count()
     clocks.window_begin()
-    times = [bracket(args.steps) for _ in range(repeats)]
+    total_ms = bracket(args.steps)
     clocks.window_end()
-    launches = (eng.launch_count() - launches0) // repeats
+    launches = eng.launch_count() - launches0
     clk = clocks.stop()
     eng.check()
-    t = torch.tensor(times, dtype=torch.float64, device=dev)
+    if args.dump_outputs and rank == 0:                     # the bracket's steps are k = 0 .. K-1
+        last = (args.steps - 1) & 1
+        dump_outputs(args.dump_outputs, wet_outs[last] if fused_wet else outs[last], off)
+    t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:
-        dist.all_reduce(t, op=dist.ReduceOp.MAX)            # every bracket: max over ranks
-    times = t.cpu().numpy()
-    total_ms = float(np.median(times))
+        dist.all_reduce(t, op=dist.ReduceOp.MAX)
+    total_ms = float(t.item())
     ms_per_step = total_ms / args.steps
     points_all = N * world
     value = points_all / (ms_per_step * 1e-3)
@@ -549,17 +568,15 @@ def main():
                    'engine.wet_ground_batch on the slot-compacted snow output, device -> pinned host copy of rows + counts, '
                    'synchronize (no pipelining across steps in this configuration)')
 
-        n_e2e = max(args.steps, 20)
         e2e_run(3)
         sync_all()
         t0 = time.perf_counter()
-        e2e_run(n_e2e)
+        e2e_run(args.steps)
         sync_all()
-        dt = (time.perf_counter() - t0) / n_e2e
-        n_sync = max(3, args.steps // 2)
+        dt = (time.perf_counter() - t0) / args.steps
         t0 = time.perf_counter()
-        e2e_sync(n_sync)
-        dt_sync = (time.perf_counter() - t0) / n_sync
+        e2e_sync(args.steps)
+        dt_sync = (time.perf_counter() - t0) / args.steps
         tt = torch.tensor([dt, dt_sync], dtype=torch.float64, device=dev)
         if world > 1:
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
@@ -570,7 +587,7 @@ def main():
             rows_out = int(host_outs[0]['counts'].sum().item())
         e2e = {'value': points_all / dt, 'unit': 'points/s', 'h2d_bytes_per_step': int(N * 20),
                'd2h_bytes_per_step': int(rows_out * 20 + B * 4 + (0 if fused_wet else B * 32)), 'ms_per_step': dt * 1e3,
-               'steps_timed': n_e2e,
+               'steps_timed': args.steps,
                'sync_call': {'value': points_all / dt_sync, 'ms_per_step': dt_sync * 1e3},
                'chunks': args.e2e_chunks, 'batches_in_flight': depth,
                'copy_out': 'kept rows by kernel' if kernel_out else 'whole slot by copy engine',
@@ -631,8 +648,7 @@ def main():
             'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f64', 'data': 'synthetic', 'config': cfg,
             'clouds_per_s': value / (64 * N_AZIMUTH), 'e2e': e2e, 'gpu_launches': int(launches), 'clocks': clk,
             'roofline': roofline, 'cpu_baseline': cpu,
-            'repeats': repeats, 'timed_region_ms': float(np.sum(times)),
-            'ms_per_step_min': float(np.min(times)) / args.steps, 'ms_per_step_max': float(np.max(times)) / args.steps,
+            'timed_region_ms': total_ms,
             'theta_label_mismatch': theta_info, 'steps_in_flight': n_streams,
             'engine': {'prepass': 'device' if device_prepass else 'DEBUG: fixed host-supplied threshold polynomial',
                        'table_particles': tinfo['n_particles'], 'table_index_bytes': tinfo['bytes'],

@@ -100,7 +100,11 @@ def test_wet_ground(oracle, gold_dir):
     assert sha(pc) == str(g['cloud_sha'])
     out = oracle.ground_water_augmentation(pc, water_height=0.001, plane=(g['plane_w'], float(g['plane_h'])),
                                            least_populated=g['ymins'])
-    assert out.dtype == np.float64 and np.array_equal(out, g['out'])
+    assert out.dtype == np.float64 and out.shape == g['out'].shape
+    assert np.array_equal(out[:, [0, 1, 2, 4]], g['out'][:, [0, 1, 2, 4]])
+    # the intensities pass through float64 np.cos / np.arccos and BLAS matrix-vector products, whose last bits depend on
+    # the host's SIMD and BLAS kernels (bit for bit on the host the fixture was made on, a few ulp apart elsewhere)
+    assert np.allclose(out[:, 3], g['out'][:, 3], rtol=1e-12, atol=0)
 
 
 def test_config1_and_config2(oracle, gold_dir):

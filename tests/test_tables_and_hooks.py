@@ -48,12 +48,10 @@ def test_dense_hook_defaults_mirror_the_dataset(monkeypatch):
         dense.OnTheFlyWeather({}, engine=object())
 
 
-@pytest.mark.skipif(not os.path.exists('/root/reference/calib/20171102_64E_S3.yaml'),
-                    reason='reference tree not mounted (build container only)')
-def test_sensor_table_equals_the_reference_yaml():
+def test_sensor_table_equals_the_reference_yaml(gold_dir):
     import yaml
     from lidar_snow_sim_b200.calib.hdl64e_s3 import HDL64E_S3
-    with open('/root/reference/calib/20171102_64E_S3.yaml') as f:
+    with open(os.path.join(gold_dir, '20171102_64E_S3.yaml')) as f:      # the reference's calib/ file, unchanged
         lasers = yaml.safe_load(f)['lasers']
     assert len(lasers) == len(HDL64E_S3) == 64
     for (lid, fd, fs, mi, vc), ref in zip(HDL64E_S3, lasers):
