@@ -296,6 +296,31 @@ LSS_API lss_status lss_voxelize_batch(lss_engine *e, const float *d_points, int 
                                       int64_t workspace_bytes, void *stream);
 LSS_API int64_t lss_voxelize_workspace_bytes(int64_t n_total, int n_clouds, int max_points_per_voxel, int max_voxels);
 
+/* ---- dynamic radius outlier removal (DROR) ----------------------------------------------------------------------------
+ * dynamic_radius_outlier_filter (lib/cadc_devkit/other/dror.py:288-334), the de-snowing filter whose snow indices the DENSE
+ * data path reads from per-frame pickles (lib/OpenPCDet/pcdet/datasets/dense/dense_dataset.py:588-616), computed on
+ * device-resident clouds, e.g. the slot-compacted output of lss_snowfall_batch.  Rule (DESIGN.md 7.4): with
+ *     sr_i = max(alpha_deg * beta * pi / 180 * sqrt(x_i^2 + y_i^2), sr_min)     float64 (dror.py:316-321)
+ *     d2_ij = ((0 + dx^2) + dy^2) + dz^2                                        float32, FLANN's L2_Simple order
+ * point i is kept iff at least k_min + 1 points j of its cloud, i included, have sqrt((double)d2_ij) < sr_i -- what the
+ * reference's k = k_min + 1 nearest-neighbour count decides (dror.py:311-334).  Integer result: exact, deterministic.
+ *   d_points        float32[n_total * n_features], n_features >= 3; xyz are read, every column is copied
+ *   d_cloud_counts  int32[n_clouds] device or NULL: valid rows per cloud slot (slot-compacted input)
+ *   h_crop_xy       float32[4] (x0, x1, y0, y1) or NULL.  Not NULL = the `crop` variant of process_dense (dror.py:238-256):
+ *                   only rows with x0 <= x <= x1 and y0 <= y <= y1 (get_cube_mask, :73-84, whose z test has no effect)
+ *                   take part; the others get code 2
+ *   d_codes         uint8[n_total]: 0 snow, 1 kept, 2 outside the crop (rows behind a cloud's count are not written)
+ *   d_out_points    float32[n_total * n_features] or NULL (codes and counts only): per cloud the kept rows in input
+ *                   order, compacted to the front of the cloud's slot, as lss_snowfall_batch lays out its output
+ *   d_out_counts    int32[n_clouds] kept rows;  d_out_n_snow  int32[n_clouds] rows with code 0
+ *   d_workspace     lss_dror_workspace_bytes(n_total, n_clouds) bytes (-1 there: no usable CUDA device)            */
+LSS_API lss_status lss_dror_batch(lss_engine *e, const float *d_points, int n_features, const int64_t *h_cloud_offsets,
+                                  const int32_t *d_cloud_counts, int n_clouds, double alpha_deg, double beta, int k_min,
+                                  double sr_min, const float *h_crop_xy, uint8_t *d_codes, float *d_out_points,
+                                  int32_t *d_out_counts, int32_t *d_out_n_snow, void *d_workspace,
+                                  int64_t workspace_bytes, void *stream);
+LSS_API int64_t lss_dror_workspace_bytes(int64_t n_total, int n_clouds);
+
 /* ---- exchange step of the sharded batch (SURVEY.md 8e, BASELINE.json configs[3]) ------------------------------------------
  * The reference has no multi-GPU augmentation; its collectives are OpenPCDet's result merging
  * (lib/OpenPCDet/pcdet/utils/commu_utils.py:77,90: all_gather of pickled, variable-size objects).  The sharded engine

@@ -84,6 +84,9 @@ SIGNATURES = [
     ('lss_voxelize_batch', _c.c_int, [_P, _P, _c.c_int, _P, _P, _c.c_int, _P, _P, _c.c_int, _c.c_int, _c.c_int, _P, _P, _P,
                                       _P, _P, _c.c_int64, _P]),
     ('lss_voxelize_workspace_bytes', _c.c_int64, [_c.c_int64, _c.c_int, _c.c_int, _c.c_int]),
+    ('lss_dror_batch', _c.c_int, [_P, _P, _c.c_int, _P, _P, _c.c_int, _c.c_double, _c.c_double, _c.c_int, _c.c_double,
+                                  _P, _P, _P, _P, _P, _P, _c.c_int64, _P]),
+    ('lss_dror_workspace_bytes', _c.c_int64, [_c.c_int64, _c.c_int]),
     ('lss_gather_push', _c.c_int, [_P, _P, _P, _P, _c.c_int, _c.c_int64, _c.c_int, _c.c_int, _P, _P, _P, _P, _c.c_int, _P]),
     ('lss_dart_throwing', _c.c_int, [_c.c_double, _c.c_double, _c.c_double, _c.c_int, _P, _P, _c.c_int64,
                                      _c.POINTER(_c.c_int64)]),

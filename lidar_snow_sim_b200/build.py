@@ -13,7 +13,7 @@ import sys
 HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, 'csrc')
 LIB = os.path.join(HERE, 'liblss_b200.so')
-SOURCES = ['api.cu', 'tables.cu', 'snowfall.cu', 'solve.cu', 'prepass.cu', 'wet_ground.cu', 'sampler.cu', 'sampler_gpu.cu', 'host_pipeline.cu', 'fog.cu', 'voxelize.cu', 'lisa.cu', 'gather.cu']
+SOURCES = ['api.cu', 'tables.cu', 'snowfall.cu', 'solve.cu', 'prepass.cu', 'wet_ground.cu', 'sampler.cu', 'sampler_gpu.cu', 'host_pipeline.cu', 'fog.cu', 'voxelize.cu', 'lisa.cu', 'gather.cu', 'dror.cu']
 # -fmad=false: float32/float64 expressions are evaluated as written (mul, then add), like NumPy on the reference host;
 # where a fused multiply-add is wanted the source says fma() / __fma_rn() explicitly.
 NVCC_FLAGS = ['-gencode', 'arch=compute_100a,code=sm_100a', '-lineinfo', '-O3', '-std=c++17', '-fmad=false',

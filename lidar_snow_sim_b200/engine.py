@@ -407,6 +407,48 @@ class SnowfallEngine:
         _lib.check(st, self.h)
         return out
 
+    def dror_batch(self, points, cloud_offsets, counts=None, alpha=0.16, beta=3.0, k_min=3, sr_min=0.04, crop_xy=None,
+                   compact=True, out=None):
+        """
+        Dynamic radius outlier removal (dynamic_radius_outlier_filter, lib/cadc_devkit/other/dror.py:288-334) of every
+        cloud of a batch, on the current stream without synchronisation.  points: CUDA float32 (N, F), F >= 3;
+        cloud_offsets: host int64 (B + 1); counts: optional CUDA int32 (B,) valid rows per cloud slot (the slot-compacted
+        output of snowfall_batch / wet_ground_batch); crop_xy: optional (x0, x1, y0, y1), the `crop` variant
+        (get_cube_mask, z ignored).  Returns dict(codes uint8 (N,) 0 snow / 1 kept / 2 outside the crop, points (N, F)
+        kept rows slot-compacted (None without `compact`), counts int32 (B,) kept rows, n_snow int32 (B,)).
+        """
+        off = np.ascontiguousarray(cloud_offsets, dtype=np.int64)
+        B = off.shape[0] - 1
+        N = int(off[-1])
+        assert points.is_cuda and points.dtype == torch.float32 and points.is_contiguous() and points.shape[0] == N
+        F = int(points.shape[1])
+        if counts is not None:
+            assert counts.is_cuda and counts.dtype == torch.int32 and counts.shape[0] == B
+        crop = None if crop_xy is None else np.ascontiguousarray(crop_xy, dtype=np.float32).reshape(4)
+        with torch.cuda.device(self.device):
+            if out is None:
+                out = {}
+            if 'codes' not in out:                             # (pass the returned dict back in as `out` to reuse the buffers)
+                out.update(codes=torch.empty((N,), dtype=torch.uint8, device=self.device),
+                           counts=torch.empty((B,), dtype=torch.int32, device=self.device),
+                           n_snow=torch.empty((B,), dtype=torch.int32, device=self.device), points=None)
+            if compact and out.get('points') is None:
+                out['points'] = torch.empty((N, F), dtype=torch.float32, device=self.device)
+            need = self.lib.lss_dror_workspace_bytes(N, B)
+            if need < 0:
+                raise RuntimeError('lss_dror_workspace_bytes failed: no usable CUDA device')
+            if getattr(self, '_ws_dror', None) is None or self._ws_dror.numel() < need:
+                self._ws_dror = torch.empty(int(need * 1.25) + 256, dtype=torch.uint8, device=self.device)
+            st = self.lib.lss_dror_batch(self.h, _ptr(points), F, _ptr(off), _ptr(counts), B, float(alpha), float(beta),
+                                         int(k_min), float(sr_min), _ptr(crop), _ptr(out['codes']),
+                                         _ptr(out['points']) if compact else None, _ptr(out['counts']),
+                                         _ptr(out['n_snow']), _ptr(self._ws_dror), int(self._ws_dror.numel()),
+                                         self._stream())
+        _lib.check(st, self.h)
+        if not compact:
+            out['points'] = None
+        return out
+
     def gather_push(self, points, counts, d_cloud_offsets, n_rows, world, rank, peer_points, peer_counts, mc_points=0,
                     mc_counts=0, blocks=0):
         """lss_gather_push on the current stream: write the kept rows of this rank's slot-compacted batch (+ counts) into

@@ -17,6 +17,7 @@ on the device once per (mode, pair) and cached.
 """
 import numpy as np
 
+from ..dror import dynamic_radius_outlier_filter
 from ..engine import default_engine
 from ..fog.simulation import ParameterSet, simulate_fog
 from ..snowfall.precompute import SNOWFALL_RATES, TERMINAL_VELOCITIES, get_fov_flag
@@ -124,6 +125,20 @@ class OnTheFlyWeather:
                 except (TypeError, ValueError):                                        # dense_dataset.py:834-837
                     pass
         return points
+
+
+def apply_dror(points, dataset_cfg, split, engine=None):
+    """The DROR / DROR++ block of `DenseDataset.__getitem__` (dense_dataset.py:588-616) without its pickles: the reference
+    reads the snow indices of the `full` variant from `training/DROR/alpha_<alpha>/all/<sensor>/<signal>/full/<id>.pkl`
+    (written offline by lib/cadc_devkit/other/dror.py); here they are computed on the device at any alpha.
+    `DROR` applies always, `DROR++` only when 'snow' is in the split name; both drop the snow rows of `points`.
+    With both keys set the second filter runs on the output of the first (the reference indexes the filtered cloud with
+    indices computed on the unfiltered one)."""
+    if 'DROR' in dataset_cfg:
+        points = points[dynamic_radius_outlier_filter(points, alpha=float(dataset_cfg['DROR']), engine=engine)]
+    if 'DROR++' in dataset_cfg and 'snow' in split:
+        points = points[dynamic_radius_outlier_filter(points, alpha=float(dataset_cfg['DROR++']), engine=engine)]
+    return points
 
 
 def foggify_cvl(points, alpha, dataset_cfg, engine=None, lut_dir=None, rng=None):
